@@ -3,6 +3,7 @@
 forced finalizeKeyFrame + createKeyFrame every 20 frames) on a synthetic 640x480 grayscale stream.
 
   python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path (one stream per GPU)
+  python bench.py ... --dump-outputs DIR                    # also write what the last timed step computed, DIR/<name>.npy
   python bench.py --impl reference --gpus N --steps K ...   # the reference's own CPU code (oracle/_ref, ENABLE_SSE build,
                                                             # 1 tracking + 4 mapping threads); the C port if _ref is absent
 
@@ -10,12 +11,20 @@ One "step" = one frame through {Frame construction, trackFrame, mapping}.  `valu
 parked in HBM (prefetch ring); `e2e` is the same loop fed from HOST buffers through the C ABI with the H2D copy of every frame
 and the D2H read of the tracking result inside the timed region.
 
-Timing: W warm-up steps, then R passes of EXACTLY K steps each on consecutive fresh frames of the stream; every pass is
-bracketed by barrier + synchronize, its time is the sum of the K per-step CUDA-event times (L2 flushed between steps), MAX
-over ranks; `value` is the MEDIAN pass (all passes are in the JSON).  With K a multiple of 20 every pass holds the same
-number of keyframe changes.  Parity is asserted in the same run (world size 1, outside the timed region): a sample of the loop's steps is replayed on the
+Timing: W warm-up steps, then ONE pass of EXACTLY K timed steps on consecutive fresh frames of the stream, per leg; the pass
+is bracketed by barrier + synchronize, its time is the sum of the K per-step CUDA-event times (L2 flushed between steps), MAX
+over ranks.  Parity is asserted in the same run (world size 1, outside the timed region): a sample of the loop's steps is replayed on the
 CPU oracle from the device's own state (identical inputs); the line carries `parity` and the run fails above 1e-4.
 Prints ONE JSON line on rank 0.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what the resident leg's LAST timed step returned to its caller, so
+that two builds run with the same arguments (hence the same seeded input stream) can be compared output for output:
+    pose_qt.npy                        float64 [7]   frameToRef (qx, qy, qz, qw, tx, ty, tz) of the tracked frame
+    track_result.npy                   float64 [20]  the other fields of lsdgpu_track_result, in the order of TRACK_FIELDS
+    new_kf_thisToParent_qts.npy        float64 [8]   the new keyframe's Sim3 output of the call (set on a keyframe change)
+    depth_<field>.npy                  float32 [h, w] every field of the current keyframe's depth map (lsdgpu_depth_download)
+The depth map is ~10 MB at 640x480; above DUMP_BUDGET the fields hold a fixed seeded sample of the pixels instead, flattened,
+and depth_sample_index.npy (float64) holds the row-major pixel index of each sampled entry.
 """
 from __future__ import annotations
 
@@ -34,14 +43,39 @@ sys.path.insert(0, ROOT)
 METRIC = "frames/sec (track+depth-update) at 640x480"
 KF_EVERY = 20
 POSE_TOL = 1e-4           # north_star: SE3 pose within 1e-4 rel on translation / rotation
+DUMP_BUDGET = 64 << 20    # bytes written by --dump-outputs at most
+TRACK_FIELDS = ("pointUsage", "lastGoodCount", "lastBadCount", "lastMeanRes", "lastResidual", "affineEstimation_a",
+                "affineEstimation_b", "diverged", "trackingWasGood", "numCalcResidualCalls", "numCalcWarpUpdateCalls",
+                "initialTrackedResidual")
 
 
 def rank_world():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1")), int(os.environ.get("LOCAL_RANK", "0"))
 
 
-def n_passes(steps: int) -> int:
-    return int(min(5, max(1, 120 // max(steps, 1))))
+def step_outputs(gs) -> dict:
+    """what GpuStream.step / lsdgpu_track_and_map handed back on the last step, plus the current keyframe's depth map"""
+    from lsd_slam_b200.abi import HYP_DTYPE
+    r = gs.tracker.last
+    out = {"pose_qt": np.array(gs.poses[-1], np.float64),
+           "track_result": np.concatenate([np.ravel(getattr(r, f)) for f in TRACK_FIELDS]).astype(np.float64),
+           "new_kf_thisToParent_qts": np.array(gs._qts, np.float64)}
+    hyp = gs.map.current()
+    fields = [f for f in HYP_DTYPE.names if f != "_pad"]
+    budget = (DUMP_BUDGET - (64 << 10)) // (4 * len(fields) + 8)          # pixels that fit, with their sample index; 64 KB for the rest
+    if hyp.size > budget:
+        idx = np.sort(np.random.default_rng(0).choice(hyp.size, budget, replace=False))
+        hyp = hyp.reshape(-1)[idx]
+        out["depth_sample_index"] = idx.astype(np.float64)
+    for f in fields:
+        out["depth_" + f] = hyp[f].astype(np.float32)
+    return out
+
+
+def write_outputs(d: str, outputs: dict):
+    os.makedirs(d, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(os.path.join(d, name + ".npy"), a)
 
 
 def nvml_index(local_rank: int) -> int:
@@ -257,8 +291,8 @@ def gpu_run(args, rank, world, local_rank):
         torch.cuda.synchronize()
 
     w, h = args.width, args.height
-    R, K, W = n_passes(args.steps), args.steps, args.warmup
-    n_frames = W + R * K + 1
+    K, W = args.steps, args.warmup
+    n_frames = W + K + 1
     # independent streams: one per GPU, seeds 1234 + 1000*rank (SURVEY 8d, config 4)
     seq, frames = render_frames(w, h, 1234 + 1000 * rank, n_frames)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")      # > 126 MB L2
@@ -285,27 +319,22 @@ def gpu_run(args, rank, world, local_rank):
         sampler.start()
         launches0 = ctx.launch_count()
         step_ms = []
-        pass_ms = []
-        wall = 0.0
-        for r in range(R):
-            barrier()
-            wall0 = time.perf_counter()
-            acc = 0.0
-            for k in range(W + 1 + r * K, W + 1 + (r + 1) * K):
-                flush.fill_(k & 0xff)                                          # L2 flush between timed steps
-                torch.cuda.synchronize()
-                ctx.timer_begin(0)
-                if leg == "e2e":
-                    gs.step(k, pinned_np[k])                                   # pinned host u8 in, pose (D2H) out
-                else:
-                    gs.step(k, stage_index=k)
-                ctx.timer_end(0)
-                ms = ctx.timer_ms(0)
-                step_ms.append(ms)
-                acc += ms
-            barrier()
-            wall += time.perf_counter() - wall0
-            pass_ms.append(acc)
+        barrier()
+        wall0 = time.perf_counter()
+        for k in range(W + 1, W + 1 + K):
+            flush.fill_(k & 0xff)                                              # L2 flush between timed steps
+            torch.cuda.synchronize()
+            ctx.timer_begin(0)
+            if leg == "e2e":
+                gs.step(k, pinned_np[k])                                       # pinned host u8 in, pose (D2H) out
+            else:
+                gs.step(k, stage_index=k)
+            ctx.timer_end(0)
+            ms = ctx.timer_ms(0)
+            step_ms.append(ms)
+        barrier()
+        wall = time.perf_counter() - wall0
+        pass_ms = [float(np.sum(step_ms))]
         clocks = sampler.stop()
         launches = ctx.launch_count() - launches0
         kms, klaunch, kbytes = ctx.track_kernel_stats(reset=2)
@@ -324,6 +353,8 @@ def gpu_run(args, rank, world, local_rank):
             per_rank = gathered
         results[leg] = dict(pass_ms=pass_max, launches=launches, clocks=clocks, wall=wall, kms=kms, klaunch=klaunch, kbytes=kbytes,
                             poses=np.array(gs.poses), p50=float(np.median(sm)), p95=float(np.percentile(sm, 95)), per_rank=per_rank)
+        if leg == "resident" and args.dump_outputs and rank == 0:
+            write_outputs(args.dump_outputs, step_outputs(gs))
         ctx.close()
     return seq, frames, results
 
@@ -339,16 +370,18 @@ def main():
     ap.add_argument("--mode", type=int, default=1, help="tracker: 1 = device-resident LM, 0 = host-driven LM")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="skip the in-run parity check (profiling runs only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank, world, local_rank = rank_world()
     metric = METRIC if (args.width, args.height) == (640, 480) else METRIC.replace("640x480", f"{args.width}x{args.height}")
     workload = f"synthetic {args.width}x{args.height} grayscale stream, full track+map loop, forced keyframe every {KF_EVERY} frames"
-    R = n_passes(args.steps)
     config = {"workload": workload, "width": args.width, "height": args.height, "pyramid_levels_tracked": "L4..L1",
               "kf_every": KF_EVERY, "streams_per_gpu": 1, "parallelism": f"{world} independent stream(s), one per GPU, no collective",
               "l2": "flushed between timed steps (256 MiB fill); per-step CUDA-event times summed",
-              "passes": R, "statistic": f"median of {R} pass(es) of exactly {args.steps} steps each (max over ranks per pass)",
+              "passes": 1, "statistic": f"one pass of exactly {args.steps} steps (max over ranks)",
               "init": "gtDepthInit (SlamSystem.cpp:831-854)",
               "e2e_input": "one 8-bit frame per step in page-locked host memory, copied H2D inside the timed step; result block read back per step"}
 
@@ -392,7 +425,7 @@ def main():
     peak_kind = "measured (MEASURED_PEAKS.json, copy burst)" if "hbm_gbs" in peaks else "fallback 6650 GB/s (B200_PROFILING.md)"
     r, e = res["resident"], res["e2e"]
     K = args.steps
-    pass_r, pass_e = float(np.median(r["pass_ms"])), float(np.median(e["pass_ms"]))
+    pass_r, pass_e = r["pass_ms"][0], e["pass_ms"][0]
     fps = world * K / (pass_r * 1e-3)
     fps_e2e = world * K / (pass_e * 1e-3)
     traffic = None
@@ -410,9 +443,9 @@ def main():
             "clocks": r["clocks"],
             "e2e": {"value": fps_e2e, "unit": "frames/s", "h2d_bytes_per_step": args.width * args.height,
                     "d2h_bytes_per_step": 144, "ms_per_step": pass_e / K, "pass_ms": e["pass_ms"]},
-            "gpu_launches": int(round(r["launches"] / R)),
+            "gpu_launches": int(r["launches"]),
             "pass_ms": r["pass_ms"],
-            "step_ms": {"p50": r["p50"], "p95": r["p95"], "wall_ms_per_step_incl_flush": 1e3 * r["wall"] / (R * K)},
+            "step_ms": {"p50": r["p50"], "p95": r["p95"], "wall_ms_per_step_incl_flush": 1e3 * r["wall"] / K},
             "per_rank": r["per_rank"], "per_rank_e2e": e["per_rank"],
             "roofline": {"kernel": "warp/residual/JtJ (SE3 tracking) kernel", "bound": "hbm", "achieved": ach, "peak": hbm_peak,
                          "unit": "GB/s", "frac": ach / hbm_peak, "traffic": traffic, "peak_kind": peak_kind,

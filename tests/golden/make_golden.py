@@ -8,8 +8,14 @@
   oracle_8f_320x240.npz     Sim3 entries from the reference-compiled library as above; keyframeMsg packing, re-activation data and
                             UndistorterPTAM from the C oracle (their reference sources need ROS message headers / OpenCV remap and
                             are not part of oracle/_ref).
+  ref_pin_320x240.json      the records of tests/test_ref_pin.py's cases computed by the reference-compiled libraries
+                            (oracle/_ref/liblsd_ref.so, liblsd_ref_sse.so); the C oracle must reproduce them.
+  reference_files.json      line count of every file of the reference tree, by path relative to its root: what
+                            tests/test_citations.py resolves the `path:line` citations against.
+The reference-generated files need the reference sources (oracle/ref_build.py builds oracle/_ref from them).
 Run:  python -m tests.golden.make_golden
 """
+import json
 import os
 import sys
 
@@ -119,7 +125,7 @@ if __name__ == "__main__":
     from oracle import pyoracle
     pyoracle.build()
     if not pyoracle.ref_available():
-        raise SystemExit("oracle/_ref is not built and /root/reference is absent: the reference-generated fixtures cannot be regenerated here")
+        raise SystemExit("oracle/_ref is not built and the reference sources are absent: the reference-generated fixtures cannot be regenerated")
     seq = synth.Sequence(320, 240, seed=1234)
     frames = {k: seq.render(k) for k in range(0, 6)}
     res = compute(Bound(pyoracle, "ref"), seq, frames)                 # the reference's own code
@@ -142,3 +148,19 @@ if __name__ == "__main__":
                                       r.affineEstimation_a, r.affineEstimation_b], np.float32)
     np.savez_compressed(os.path.join(HERE, "oracle_8f_320x240.npz"), **res)
     print({k: v.shape for k, v in res.items()})
+
+    from tests import test_ref_pin
+    pin_frames = {k: seq.render(k) for k in range(0, 26)}
+    with open(os.path.join(HERE, "ref_pin_320x240.json"), "w") as f:
+        json.dump(test_ref_pin.reference_records(seq, pin_frames), f, indent=1)
+
+    from oracle import ref_build
+    if ref_build.available():
+        ref_root = os.path.dirname(ref_build.REF)
+        lines = {}
+        for root, _, files in os.walk(ref_root):
+            for name in files:
+                p = os.path.join(root, name)
+                lines[os.path.relpath(p, ref_root)] = sum(1 for _ in open(p, errors="ignore"))
+        with open(os.path.join(HERE, "reference_files.json"), "w") as f:
+            json.dump(dict(sorted(lines.items())), f, indent=1)

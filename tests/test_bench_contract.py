@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -48,14 +50,13 @@ def _fake_gpu_run_factory(bench):
     import numpy as np
 
     def fake_gpu_run(args, rank, world, local_rank):
-        R = bench.n_passes(args.steps)
-        n = args.warmup + R * args.steps
+        n = args.warmup + args.steps
         seq, frames = bench.render_frames(args.width, args.height, 1234, n + 1)
-        pr = [{"rank": 0, "sum_ms": 2.0 * R, "p50": 0.2, "p95": 0.22, "max_step_ms": 0.3, "argmax_step": 1, "pass_ms": [2.0] * R,
+        pr = [{"rank": 0, "sum_ms": 2.0, "p50": 0.2, "p95": 0.22, "max_step_ms": 0.3, "argmax_step": 1, "pass_ms": [2.0],
                "sm_mhz": 1965.0, "reasons": [], "pinned_cores": None}]
-        leg = dict(pass_ms=[2.0] * R, launches=53 * R, clocks={"sm_mhz": 1965.0, "sm_max_mhz": 1965.0, "reasons": [], "samples": 5}, wall=0.1,
+        leg = dict(pass_ms=[2.0], launches=53, clocks={"sm_mhz": 1965.0, "sm_max_mhz": 1965.0, "reasons": [], "samples": 5}, wall=0.1,
                    kms=1.1, klaunch=10, kbytes=1.1e8, poses=np.zeros((n, 7)), p50=0.2, p95=0.22, per_rank=pr)
-        return seq, frames, {"resident": leg, "e2e": dict(leg, pass_ms=[2.2] * R)}
+        return seq, frames, {"resident": leg, "e2e": dict(leg, pass_ms=[2.2])}
     return fake_gpu_run
 
 
@@ -78,7 +79,6 @@ def test_product_arm_line_contract_with_mocked_device_results(monkeypatch, capsy
     monkeypatch.setattr(bench, "gpu_run", _fake_gpu_run_factory(bench))
     monkeypatch.setattr(bench, "parity_leg", _fake_parity_leg_factory(bench, 2e-5))
     monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "20", "--warmup", "3"])
-    monkeypatch.setattr(bench, "n_passes", lambda steps: 1)
     bench.main()
     lines = [ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")]
     assert len(lines) == 1
@@ -103,15 +103,37 @@ def test_product_arm_line_contract_with_mocked_device_results(monkeypatch, capsy
 
 def test_product_arm_fails_when_parity_is_off(monkeypatch, capsys):
     """a pose 3e-4 away from the oracle on a replayed step: the line still prints (parity.ok false), the process exits non-zero"""
-    import pytest
     sys.path.insert(0, ROOT)
     import bench
     monkeypatch.setattr(bench, "gpu_run", _fake_gpu_run_factory(bench))
     monkeypatch.setattr(bench, "parity_leg", _fake_parity_leg_factory(bench, 3e-4))
     monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "4", "--warmup", "3", "--no-cpu-baseline"])
-    monkeypatch.setattr(bench, "n_passes", lambda steps: 1)
     with pytest.raises(SystemExit) as ei:
         bench.main()
     assert ei.value.code == 3
     d = json.loads([ln for ln in capsys.readouterr().out.splitlines() if ln.startswith("{")][0])
     assert d["parity"]["ok"] is False
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_identical_across_runs(tmp_path):
+    """--dump-outputs writes the last timed step's results as float32 / float64 .npy files within 64 MB; two runs with the same
+    arguments see the same seeded stream and must write the same arrays bit for bit (the kernels use no float atomics)"""
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        d = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "6", "--warmup", "3", "--width", "320", "--height", "240",
+                            "--no-cpu-baseline", "--no-parity", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 6
+        assert sum(p.stat().st_size for p in d.iterdir()) <= 64 << 20
+        dumps.append({p.stem: np.load(p) for p in d.glob("*.npy")})
+    a, b = dumps
+    assert {"pose_qt", "track_result", "new_kf_thisToParent_qts", "depth_isValid", "depth_idepth", "depth_idepth_var"} <= set(a)
+    assert set(a) == set(b)
+    for name, x in a.items():
+        assert x.dtype in (np.float32, np.float64), name
+        assert x.tobytes() == b[name].tobytes(), name
+    assert a["pose_qt"].shape == (7,) and np.isfinite(a["pose_qt"]).all() and a["depth_idepth"].shape == (240, 320)
+    assert a["depth_isValid"].sum() > 10000
