@@ -30,7 +30,8 @@ extern "C" {
 
 #define LSDGPU_LEVELS 5                 /* PYRAMID_LEVELS, util/settings.h:106 */
 /* 2: additive over 1 -- lsdgpu_get_globals, lsdgpu_depth_update_keyframe_refs (lsdgpu_ref_desc), lsdgpu_seq_sum_f32,
- *    lsdgpu_peer_export / _attach / _detach; contexts are thread-safe (per-context mutex).  No existing signature changed. */
+ *    lsdgpu_peer_export / _attach / _detach, lsdgpu_map_export_points (lsdgpu_map_filter, lsdgpu_map_point); contexts are
+ *    thread-safe (per-context mutex).  No existing signature changed. */
 #define LSDGPU_ABI_VERSION 2
 
 typedef struct lsdgpu_ctx lsdgpu_ctx;
@@ -207,6 +208,22 @@ typedef struct { float idepth; float idepth_var; unsigned char color[4]; } lsdgp
 /* the packing loop of ROSOutput3DWrapper::publishKeyframe (ROSOutput3DWrapper.cpp:91-110) for level `publish_level`:
  * out receives (w >> level) * (h >> level) records, one device-to-host copy in wire layout */
 int lsdgpu_keyframe_pack_pointcloud(lsdgpu_ctx* ctx, int kf_id, int publish_level, lsdgpu_input_point_dense* out);
+/* The map as lsd_slam_viewer saves it (pc.ply), for many resident keyframes in one call: the point filter and world-frame transform
+ * of KeyFrameDisplay::flushPC (lsd_slam_viewer/src/KeyFrameDisplay.cpp:269-340) applied to what lsdgpu_keyframe_pack_pointcloud
+ * would publish for each keyframe (idepth, idepthVar and image of `publish_level`).  camToWorld_qts[8*i..] = the caller's
+ * getScaledCamToWorld() of kf_ids[i] (unit quaternion x,y,z,w, translation, scale), cast to the float Sophus storage as
+ * ROSOutput3DWrapper.cpp:85 does.  Records follow kf_ids order, then y, then x; counts_out[i] = points of keyframe i.
+ * out == NULL: counts only.  Errors (nothing written): unknown id, a keyframe without depth, bad level, total > capacity.
+ * sparsifyFactor > 1 (a rand() draw per pixel) is not offered; keyframe selection (cutFirstNKf) is the caller's list. */
+/* the point filter of lsd_slam_viewer's KeyFrameDisplay::flushPC (KeyFrameDisplay.cpp:274-307); viewer defaults
+ * settings.cpp:36-38 = (1, 1, 5), under ROS cfg/LSDSLAMViewerParams.cfg:20-22 = (10^-3, 10^-1, 7) */
+typedef struct { float scaledDepthVarTH, absDepthVarTH; int minNearSupport; } lsdgpu_map_filter;
+/* one vertex record of pc.ply (KeyFrameDisplay.cpp:328-333, header KeyFrameGraphDisplay.cpp:75-82) */
+typedef struct { float x, y, z, intensity; } lsdgpu_map_point;
+int lsdgpu_map_export_points(lsdgpu_ctx* ctx, int n_kf, const int* kf_ids, const double* camToWorld_qts /* 8*n_kf */,
+                             int publish_level, const lsdgpu_map_filter* f,
+                             lsdgpu_map_point* out /* NULL: counts only */, long long capacity,
+                             int* counts_out /* n_kf, may be NULL */, long long* total_out);
 /* Frame::takeReActivationData(currentDepthMap), DataStructures/Frame.cpp:107-145: snapshot of the ACTIVE depth map into the
  * keyframe's idepth_reAct / idepthVar_reAct / validity_reAct -- kept on the device.  lsdgpu_depth_finalize_keyframe calls it
  * (DepthMap.cpp:1387); exposed for re-activation bookkeeping outside finalize. */

@@ -91,6 +91,29 @@ class Sim3EvalResult(C.Structure):
                 ("pointUsage", C.c_float), ("affine_a_lastIt", C.c_float), ("affine_b_lastIt", C.c_float)]
 
 
+class MapFilter(C.Structure):
+    """lsdgpu_map_filter: the point filter of lsd_slam_viewer's KeyFrameDisplay::flushPC (KeyFrameDisplay.cpp:274-307)"""
+    _fields_ = [("scaledDepthVarTH", C.c_float), ("absDepthVarTH", C.c_float), ("minNearSupport", C.c_int)]
+
+
+def write_ply(path, points: np.ndarray) -> None:
+    """Write (N, 4) float32 map points (x, y, z, intensity) as the binary PLY of lsd_slam_viewer's KeyFrameGraphDisplay::draw
+    (header KeyFrameGraphDisplay.cpp:75-82, records KeyFrameDisplay.cpp:328-333).  The viewer's copy loop (:85) also appends one
+    stray 0xFF byte after the last record (it writes the EOF of f3.get()); that byte is not written here."""
+    pts = np.ascontiguousarray(points, np.float32).reshape(-1, 4)
+    header = ("ply\n"
+              "format binary_little_endian 1.0\n"
+              f"element vertex {pts.shape[0]}\n"
+              "property float x\n"
+              "property float y\n"
+              "property float z\n"
+              "property float intensity\n"
+              "end_header\n")
+    with open(path, "wb") as f:
+        f.write(header.encode("ascii"))
+        f.write(pts.astype("<f4", copy=False).tobytes())
+
+
 SYMBOLS = [
     ("lsdgpu_create", C.c_int, [C.c_int, C.c_int, C.c_int, _fp, C.c_int, C.POINTER(_vp)]),
     ("lsdgpu_destroy", None, [_vp]),
@@ -130,6 +153,8 @@ SYMBOLS = [
     ("lsdgpu_undistort_u8", C.c_int, [_vp, C.POINTER(C.c_uint8), C.POINTER(C.c_uint8)]),
     ("lsdgpu_frame_upload_distorted_u8", C.c_int, [_vp, C.c_int, C.POINTER(C.c_uint8)]),
     ("lsdgpu_keyframe_pack_pointcloud", C.c_int, [_vp, C.c_int, C.c_int, _vp]),
+    ("lsdgpu_map_export_points", C.c_int, [_vp, C.c_int, _ip, _dp, C.c_int, C.POINTER(MapFilter), _vp, C.c_longlong, _ip,
+                                           C.POINTER(C.c_longlong)]),
     ("lsdgpu_frame_take_reactivation_data", C.c_int, [_vp, C.c_int]),
     ("lsdgpu_frame_download_reactivation_data", C.c_int, [_vp, C.c_int, _fp, _fp, C.POINTER(C.c_uint8)]),
     ("lsdgpu_depth_set_from_existing_kf", C.c_int, [_vp, C.c_int]),
@@ -403,6 +428,26 @@ class Context:
         out = np.zeros(n, POINT_DENSE)
         self._ck(self.L.lsdgpu_keyframe_pack_pointcloud(self.ptr, kf_id, level, out.ctypes.data_as(_vp)))
         return out
+
+    def export_map(self, kf_ids, cam_to_world_qts, level: int = 0, scaled_th: float = 1e-3, abs_th: float = 1e-1,
+                   min_near_support: int = 7):
+        """The map as lsd_slam_viewer saves it (KeyFrameDisplay::flushPC over the listed keyframes, lsdgpu_map_export_points):
+        returns (points (N, 4) float32 = x, y, z, intensity in world frame, counts per keyframe).  cam_to_world_qts: one
+        getScaledCamToWorld() per keyframe as (qx, qy, qz, qw, tx, ty, tz, scale).  Defaults: the ROS viewer parameters
+        (cfg/LSDSLAMViewerParams.cfg:20-22); the viewer's built-in defaults are (1, 1, 5) (settings.cpp:36-38)."""
+        ids = np.ascontiguousarray(kf_ids, np.int32).reshape(-1)
+        qts = np.ascontiguousarray(cam_to_world_qts, np.float64).reshape(-1, 8)
+        if qts.shape[0] != ids.size:
+            raise ValueError("one camToWorld per keyframe")
+        f = MapFilter(scaled_th, abs_th, min_near_support)
+        counts = np.zeros(ids.size, np.int32)
+        total = C.c_longlong(0)
+        args = (self.ptr, ids.size, ids.ctypes.data_as(_ip), qts.ctypes.data_as(_dp), level, C.byref(f))
+        self._ck(self.L.lsdgpu_map_export_points(*args, None, 0, counts.ctypes.data_as(_ip), C.byref(total)))
+        points = np.empty((total.value, 4), np.float32)
+        self._ck(self.L.lsdgpu_map_export_points(*args, points.ctypes.data_as(_vp), total.value, counts.ctypes.data_as(_ip),
+                                                 C.byref(total)))
+        return points, counts
 
     def take_reactivation_data(self, kf_id: int):
         self._ck(self.L.lsdgpu_frame_take_reactivation_data(self.ptr, kf_id))

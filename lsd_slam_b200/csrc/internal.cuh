@@ -154,6 +154,7 @@ struct lsdgpu_ctx {
     int rawW = 0, rawH = 0;
     bool undistorterSet = false;
     uint32_t* dPacked = nullptr;         // keyframeMsg.pointcloud staging: w*h InputPointDense records (device)
+    struct MapStaging* map = nullptr;    // lsdgpu_map_export_points staging (mapexport.cuh): its own allocation, made at the first export
     int trackGrid = 148;                 // launch shape of the persistent tracker (set by trackPersistentSetup): one CTA per SM
     int trackG[LSD_LEVELS] = { 1, 1, 1, 1, 1 };          // CTAs taking part in the evaluations of each level
     unsigned int* trkSync = nullptr;     // per-level barrier counters + level records of the persistent tracker (TP_SYNC_WORDS)

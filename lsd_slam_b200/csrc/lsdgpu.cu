@@ -10,6 +10,7 @@
 #include "perma.cuh"
 #include "sim3.cuh"
 #include "output.cuh"
+#include "mapexport.cuh"
 
 #include <algorithm>
 #include <stdlib.h>
@@ -198,6 +199,7 @@ extern "C" int lsdgpu_create(int device, int width, int height, const float K[9]
 }
 
 static void peerCloseAll(lsdgpu_ctx* ctx);
+static void mapStagingFree(lsdgpu_ctx* ctx);
 
 extern "C" void lsdgpu_destroy(lsdgpu_ctx* ctx)
 {
@@ -205,6 +207,7 @@ extern "C" void lsdgpu_destroy(lsdgpu_ctx* ctx)
     cudaSetDevice(ctx->device);
     if (ctx->stream) cudaStreamSynchronize(ctx->stream);
     peerCloseAll(ctx);
+    mapStagingFree(ctx);
     cudaFree(ctx->arena);
     if (ctx->stageRing) cudaFree(ctx->stageRing);
     if (ctx->dRemapX) cudaFree(ctx->dRemapX);
@@ -1578,6 +1581,180 @@ extern "C" int lsdgpu_keyframe_pack_pointcloud(lsdgpu_ctx* ctx, int kf_id, int p
     LSD_CHECK(ctx, cudaGetLastError());
     LSD_CHECK(ctx, cudaMemcpyAsync(out, ctx->dPacked, (size_t)n * 12, cudaMemcpyDeviceToHost, ctx->stream));
     LSD_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------
+// map export: KeyFrameDisplay::flushPC over many resident keyframes (mapexport.cuh)
+// ------------------------------------------------------------------------------------------------------
+// Device staging outside the arena, so that contexts which never export keep the arena layout the peer-sharded tracker
+// requires to be identical on every rank.  The record buffers are sized once (two chunks of MAP_CHUNK worst-case
+// keyframes); the per-keyframe index arrays are sized for max(max_frames, n_kf) and only grow when a call lists more keyframes.
+struct MapStaging {
+    int kfCap = 0, bandCap = 0;
+    MapKf* dKf = nullptr;
+    MapKf* hKf = nullptr;                // pinned
+    int* dCta = nullptr;                 // [kfCap * bandCap] per-CTA counts
+    long long* dOff = nullptr;           // [kfCap * bandCap] output offsets
+    int* dKfCount = nullptr;             // [kfCap]
+    long long* dTotal = nullptr;
+    int* hKfCount = nullptr;             // pinned [kfCap]
+    long long* hTotal = nullptr;         // pinned
+    float4* dRec[2] = { nullptr, nullptr };
+    cudaStream_t copy = nullptr;         // device-to-host copies of the records, overlapping the next chunk's kernel
+    cudaEvent_t kernDone[2] = { nullptr, nullptr }, copyDone[2] = { nullptr, nullptr };
+};
+
+static int mapBandRows(int W)
+{   // (rows + 2) x W floats of shared memory: at most 48 KB where the width allows it, at most 16 rows
+    return std::max(1, std::min(16, 48 * 1024 / (4 * std::max(W, 1)) - 2));
+}
+
+static void mapFreeIndex(MapStaging* m)
+{
+    cudaFree(m->dKf); cudaFree(m->dCta); cudaFree(m->dOff); cudaFree(m->dKfCount);
+    cudaFreeHost(m->hKf); cudaFreeHost(m->hKfCount);
+    m->dKf = nullptr; m->dCta = nullptr; m->dOff = nullptr; m->dKfCount = nullptr; m->hKf = nullptr; m->hKfCount = nullptr;
+    m->kfCap = 0;
+}
+
+static void mapStagingFree(lsdgpu_ctx* ctx)
+{
+    MapStaging* m = ctx->map;
+    if (!m) return;
+    if (m->copy) cudaStreamSynchronize(m->copy);
+    mapFreeIndex(m);
+    cudaFree(m->dTotal); cudaFreeHost(m->hTotal);
+    cudaFree(m->dRec[0]); cudaFree(m->dRec[1]);
+    for (int b = 0; b < 2; b++) {
+        if (m->kernDone[b]) cudaEventDestroy(m->kernDone[b]);
+        if (m->copyDone[b]) cudaEventDestroy(m->copyDone[b]);
+    }
+    if (m->copy) cudaStreamDestroy(m->copy);
+    delete m;
+    ctx->map = nullptr;
+}
+
+static int mapReserve(lsdgpu_ctx* ctx, int n_kf)
+{
+    if (!ctx->map) {
+        MapStaging* m = new (std::nothrow) MapStaging();
+        if (!m) return lsd_fail(ctx, "out of host memory");
+        ctx->map = m;
+        int bands = 0;
+        for (int l = 0; l < LSD_LEVELS; l++) {
+            const int W = ctx->w >> l, H = ctx->h >> l, r = mapBandRows(W);
+            if (W >= 3 && H >= 3) bands = std::max(bands, divUp(H - 2, r));
+        }
+        m->bandCap = std::max(bands, 1);
+        const size_t recs = (size_t)MAP_CHUNK * ctx->w * ctx->h;
+        LSD_CHECK(ctx, cudaMalloc((void**)&m->dRec[0], recs * sizeof(float4)));
+        LSD_CHECK(ctx, cudaMalloc((void**)&m->dRec[1], recs * sizeof(float4)));
+        LSD_CHECK(ctx, cudaMalloc((void**)&m->dTotal, sizeof(long long)));
+        LSD_CHECK(ctx, cudaHostAlloc((void**)&m->hTotal, sizeof(long long), cudaHostAllocDefault));
+        LSD_CHECK(ctx, cudaStreamCreateWithFlags(&m->copy, cudaStreamNonBlocking));
+        for (int b = 0; b < 2; b++) {
+            LSD_CHECK(ctx, cudaEventCreateWithFlags(&m->kernDone[b], cudaEventDisableTiming));
+            LSD_CHECK(ctx, cudaEventCreateWithFlags(&m->copyDone[b], cudaEventDisableTiming));
+        }
+        const size_t smem = (size_t)(mapBandRows(ctx->w) + 2) * ctx->w * 4;
+        if (smem > 48 * 1024) {
+            LSD_CHECK(ctx, cudaFuncSetAttribute(k_map_points<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            LSD_CHECK(ctx, cudaFuncSetAttribute(k_map_points<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        }
+    }
+    MapStaging* m = ctx->map;
+    if (n_kf <= m->kfCap) return 0;
+    mapFreeIndex(m);
+    const int cap = std::max(n_kf, (int)ctx->slots.size());
+    const size_t nc = (size_t)cap * m->bandCap;
+    LSD_CHECK(ctx, cudaMalloc((void**)&m->dKf, (size_t)cap * sizeof(MapKf)));
+    LSD_CHECK(ctx, cudaMalloc((void**)&m->dCta, nc * sizeof(int)));
+    LSD_CHECK(ctx, cudaMalloc((void**)&m->dOff, nc * sizeof(long long)));
+    LSD_CHECK(ctx, cudaMalloc((void**)&m->dKfCount, (size_t)cap * sizeof(int)));
+    LSD_CHECK(ctx, cudaHostAlloc((void**)&m->hKf, (size_t)cap * sizeof(MapKf), cudaHostAllocDefault));
+    LSD_CHECK(ctx, cudaHostAlloc((void**)&m->hKfCount, (size_t)cap * sizeof(int), cudaHostAllocDefault));
+    m->kfCap = cap;
+    return 0;
+}
+
+extern "C" int lsdgpu_map_export_points(lsdgpu_ctx* ctx, int n_kf, const int* kf_ids, const double* camToWorld_qts, int publish_level,
+                                        const lsdgpu_map_filter* f, lsdgpu_map_point* out, long long capacity, int* counts_out,
+                                        long long* total_out)
+{ LSD_LOCK(ctx);
+    LSD_CHECK(ctx, cudaSetDevice(ctx->device));
+    if (n_kf < 0 || !f || (n_kf > 0 && (!kf_ids || !camToWorld_qts)) || (out && capacity < 0)) return lsd_fail(ctx, "bad arguments");
+    if (publish_level < 0 || publish_level >= LSD_LEVELS) return lsd_fail(ctx, "bad level");
+    std::vector<FrameSlot*> kfs(n_kf);
+    for (int i = 0; i < n_kf; i++) {
+        kfs[i] = findSlot(ctx, kf_ids[i]);
+        if (!kfs[i]) return lsd_fail(ctx, "unknown keyframe id");
+        if (!kfs[i]->hasDepth) return lsd_fail(ctx, "keyframe has no depth");
+    }
+    const LevelCam& cam = ctx->cam[publish_level];
+    MapParams p;
+    p.W = cam.w; p.H = cam.h;
+    p.bandRows = mapBandRows(p.W);
+    p.nBands = (p.W >= 3 && p.H >= 3) ? divUp(p.H - 2, p.bandRows) : 0;
+    p.fxi = 1 / cam.fx; p.fyi = 1 / cam.fy; p.cxi = -cam.cx / cam.fx; p.cyi = -cam.cy / cam.fy;   // KeyFrameDisplay.cpp:75-78
+    p.scaledTH = f->scaledDepthVarTH; p.absTH = f->absDepthVarTH; p.minNearSupport = f->minNearSupport;
+    if (n_kf == 0 || p.nBands == 0) {
+        if (counts_out) for (int i = 0; i < n_kf; i++) counts_out[i] = 0;
+        if (total_out) *total_out = 0;
+        return 0;
+    }
+    for (FrameSlot* s : kfs) {                                      // f->idepth(publishLvl), ROSOutput3DWrapper.cpp:96-97
+        int r = ensureIdepthPyramid(ctx, s);
+        if (r) return r;
+    }
+    int r = mapReserve(ctx, n_kf);
+    if (r) return r;
+    MapStaging* m = ctx->map;
+    for (int i = 0; i < n_kf; i++) {
+        MapKf& k = m->hKf[i];
+        k.idepth = kfs[i]->idepth[publish_level]; k.var = kfs[i]->idepthVar[publish_level]; k.img = kfs[i]->image[publish_level];
+        // getScaledCamToWorld().cast<float>() (ROSOutput3DWrapper.cpp:85): the Sophus storage, quaternion with |q| = scale
+        const double* a = camToWorld_qts + 8 * (size_t)i;
+        float q[4];
+        for (int j = 0; j < 4; j++) q[j] = (float)(a[j] * a[7]);
+        for (int j = 0; j < 3; j++) k.t[j] = (float)a[4 + j];
+        k.scale = sqrtf((q[0] * q[0] + q[1] * q[1]) + (q[2] * q[2] + q[3] * q[3]));       // Eigen's tree reduction
+        for (int j = 0; j < 4; j++) k.nq[j] = q[j] / k.scale;
+    }
+    LSD_CHECK(ctx, cudaMemcpyAsync(m->dKf, m->hKf, (size_t)n_kf * sizeof(MapKf), cudaMemcpyHostToDevice, ctx->stream));
+    const size_t smem = (size_t)(p.bandRows + 2) * p.W * 4;
+    for (int b = 0; b < n_kf; b += 65535) {
+        k_map_points<false><<<dim3(p.nBands, std::min(65535, n_kf - b)), MAP_THREADS, smem, ctx->stream>>>(m->dKf, b, p, m->dCta, nullptr, 0, nullptr);
+        LAUNCH(ctx);
+    }
+    k_map_scan<<<1, 1024, 0, ctx->stream>>>(m->dCta, n_kf * p.nBands, p.nBands, m->dOff, m->dKfCount, m->dTotal);
+    LAUNCH(ctx);
+    LSD_CHECK(ctx, cudaGetLastError());
+    LSD_CHECK(ctx, cudaMemcpyAsync(m->hKfCount, m->dKfCount, (size_t)n_kf * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    LSD_CHECK(ctx, cudaMemcpyAsync(m->hTotal, m->dTotal, sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+    LSD_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    const long long total = *m->hTotal;
+    if (out && total > capacity) return lsd_fail(ctx, "map export: capacity is smaller than the number of points");
+    if (out && total > 0) {
+        std::vector<long long> kfOff(n_kf + 1, 0);
+        for (int i = 0; i < n_kf; i++) kfOff[i + 1] = kfOff[i] + m->hKfCount[i];
+        for (int c = 0, ci = 0; c < n_kf; c += MAP_CHUNK, ci++) {
+            const int e = std::min(c + MAP_CHUNK, n_kf), b = ci & 1;
+            if (ci >= 2) LSD_CHECK(ctx, cudaStreamWaitEvent(ctx->stream, m->copyDone[b], 0));     // buffer b still being copied out
+            k_map_points<true><<<dim3(p.nBands, e - c), MAP_THREADS, smem, ctx->stream>>>(m->dKf, c, p, nullptr, m->dOff, kfOff[c], m->dRec[b]);
+            LAUNCH(ctx);
+            LSD_CHECK(ctx, cudaGetLastError());
+            LSD_CHECK(ctx, cudaEventRecord(m->kernDone[b], ctx->stream));
+            LSD_CHECK(ctx, cudaStreamWaitEvent(m->copy, m->kernDone[b], 0));
+            const long long n = kfOff[e] - kfOff[c];
+            if (n) LSD_CHECK(ctx, cudaMemcpyAsync(out + kfOff[c], m->dRec[b], (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, m->copy));
+            LSD_CHECK(ctx, cudaEventRecord(m->copyDone[b], m->copy));
+        }
+        LSD_CHECK(ctx, cudaStreamSynchronize(m->copy));
+        LSD_CHECK(ctx, cudaStreamSynchronize(ctx->stream));
+    }
+    if (counts_out) memcpy(counts_out, m->hKfCount, (size_t)n_kf * sizeof(int));
+    if (total_out) *total_out = total;
     return 0;
 }
 

@@ -4,6 +4,7 @@
 // Prints one line per tracked frame: "<id> qx qy qz qw tx ty tz good".
 #include <cstdio>
 #include <cstdlib>
+#include <sstream>
 #include <string>
 #include <vector>
 
@@ -86,6 +87,14 @@ int main(int argc, char** argv)
                 prev = fr;
                 if (!early) early = fr;
             }
+        }
+        {                                                                  // the saved map of every keyframe (pc.ply)
+            std::vector<Frame*> kfs;
+            for (auto& o : oldKeyframes) kfs.push_back(o.get());
+            kfs.push_back(kf.get());
+            std::ostringstream ply;
+            const long long pts = writeMapPly(dev, kfs, ply);
+            std::fprintf(stderr, "host_demo: map of %zu keyframes: %lld points, %zu PLY bytes\n", kfs.size(), pts, ply.str().size());
         }
         map.invalidate();
     } catch (const std::exception& e) {

@@ -394,4 +394,31 @@ void DepthMap::download(std::vector<lsdgpu_hyp>& out)
     dev_.check(lsdgpu_depth_download(dev_.raw(), out.data()), "DepthMap::download");
 }
 
+long long writeMapPly(DeviceContext& dev, const std::vector<Frame*>& keyframes, std::ostream& out, int publishLevel,
+                      const lsdgpu_map_filter* f)
+{
+    const lsdgpu_map_filter rosDefaults = { 1e-3f, 1e-1f, 7 };
+    if (!f) f = &rosDefaults;
+    const int n = (int)keyframes.size();
+    std::vector<int> ids(n);
+    std::vector<double> qts(8 * (size_t)n);
+    for (int i = 0; i < n; i++) {
+        ids[i] = keyframes[i]->id();
+        const Sim3 c = keyframes[i]->getScaledCamToWorld();
+        for (int j = 0; j < 4; j++) qts[8 * i + j] = c.q[j];
+        for (int j = 0; j < 3; j++) qts[8 * i + 4 + j] = c.t[j];
+        qts[8 * i + 7] = c.s;
+    }
+    long long total = 0;
+    dev.check(lsdgpu_map_export_points(dev.raw(), n, ids.data(), qts.data(), publishLevel, f, nullptr, 0, nullptr, &total),
+              "map export (count)");
+    std::vector<lsdgpu_map_point> pts((size_t)total);
+    dev.check(lsdgpu_map_export_points(dev.raw(), n, ids.data(), qts.data(), publishLevel, f, pts.data(), total, nullptr, &total),
+              "map export");
+    out << "ply\n" << "format binary_little_endian 1.0\n" << "element vertex " << total << "\n"
+        << "property float x\n" << "property float y\n" << "property float z\n" << "property float intensity\n" << "end_header\n";
+    out.write(reinterpret_cast<const char*>(pts.data()), (std::streamsize)(pts.size() * sizeof(lsdgpu_map_point)));
+    return total;
+}
+
 }  // namespace lsd_slam

@@ -13,6 +13,7 @@
 
 #include <deque>
 #include <memory>
+#include <ostream>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -242,5 +243,12 @@ private:
     DeviceContext& dev_;
     int width_, height_;
 };
+
+// lsd_slam_viewer's saved map (pc.ply, KeyFrameGraphDisplay::draw, KeyFrameGraphDisplay.cpp:63-93) of the given keyframes, computed
+// on the device by lsdgpu_map_export_points from each keyframe's getScaledCamToWorld(): the binary PLY header of :75-82 followed by
+// one (x, y, z, intensity) float record per point (without the stray trailing byte of the viewer's copy loop, :85).
+// f == nullptr: the ROS viewer parameters (cfg/LSDSLAMViewerParams.cfg:20-22).  Returns the number of points.
+long long writeMapPly(DeviceContext& dev, const std::vector<Frame*>& keyframes, std::ostream& out, int publishLevel = 0,
+                      const lsdgpu_map_filter* f = nullptr);
 
 }  // namespace lsd_slam

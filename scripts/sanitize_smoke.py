@@ -64,3 +64,15 @@ raw = np.random.default_rng(1).integers(0, 256, (128, 192)).astype(np.uint8)
 ctx2.undistort(raw); ctx2.upload_distorted(0, raw)
 ctx2.close(); ctx.close()
 print("sanitize run (8f rows) ok")
+
+# map export (lsdgpu_map_export_points): count, scan and write kernels over more keyframes than one staging chunk, levels 0-2
+ctx = abi.Context(160, 112, seq.K, max_frames=8)
+for k in (0, 3, 6):
+    ctx.upload(k, fr[k][0]); ctx.set_depth_gt(k, fr[k][1])
+ids = [0, 3, 6] * 4
+qts = np.array([np.concatenate([seq.frame_to_ref_qt(k), [1.0 + 0.1 * i]]) for i, k in enumerate(ids)])
+for lvl in (0, 1, 2):
+    ctx.export_map(ids, qts, lvl, 1.0, 1.0, 5)
+    ctx.export_map(ids, qts, lvl)
+ctx.close()
+print("sanitize run (map export) ok")
